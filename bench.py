@@ -387,8 +387,46 @@ def parity_check(cx, rule, G, n, d, f, out, z=1.5):
     return res
 
 
-def run_config(cx, rule, n, d, f, dtype, steps, warmup, want_e2e=False, e2e_steps=3, z=1.5, check=True):
-    """One benchmark configuration on the current process group: returns the fields of a bench record."""
+DUMP_BYTES = 64_000_000
+
+
+def last_step_outputs(cx, rule, G, out, d):
+    """What a caller of the timed path receives from its last step, on every rank: the per-column outputs gathered
+    to full length D (float32 device tensors), and the selected indices."""
+    import torch
+    if rule == "Krum":
+        cols, picks = {"aggregate": G[out]}, {"krum_index": torch.tensor([out])}       # defences.krum returns the row G[idx]
+    elif rule == "Bulyan":
+        cols, picks = {"aggregate": out[0]}, {"bulyan_selection": out[1]}
+    else:
+        cols, picks = {"crafted" if rule == "ALIE" else "aggregate": out}, {}
+    cols = {k: cx.agg.gather_output(v.float(), d) for k, v in cols.items()}
+    return cols, picks
+
+
+def write_outputs(dirname, cols, picks, budget=DUMP_BYTES):
+    """Writes DIR/<name>.npy: the per-column outputs `cols` (equal-length vectors) as float32, the indices `picks` as
+    float64, `budget` bytes in all.  When the vectors do not fit, each is cut to the same seeded sample of columns (the
+    same columns for the same D in every run), and the sampled column numbers go to DIR/columns.npy."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    picks = {name: torch.as_tensor(v).cpu().numpy().astype(np.float64) for name, v in picks.items()}
+    room = budget - sum(v.nbytes for v in picks.values()) - 128 * (len(cols) + len(picks) + 1)   # 128: .npy header
+    d = next(iter(cols.values())).numel() if cols else 0
+    if 4 * d * len(cols) > room:
+        pos = np.unique(np.random.default_rng(20261017).integers(0, d, room // (4 * len(cols) + 8)))
+        picks["columns"] = pos.astype(np.float64)
+        cols = {name: v[torch.from_numpy(pos).to(v.device)] for name, v in cols.items()}
+    for name, v in cols.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), v.float().cpu().numpy())
+    for name, v in picks.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), v)
+
+
+def run_config(cx, rule, n, d, f, dtype, steps, warmup, want_e2e=False, e2e_steps=3, z=1.5, check=True, dump_dir=None):
+    """One benchmark configuration on the current process group: returns the fields of a bench record.  `dump_dir`:
+    rank 0 writes the outputs of the last timed step there (`write_outputs`)."""
     import torch
     import torch.distributed as dist
     from attacking_federate_learning_b200 import _native as nat, defences as D
@@ -438,6 +476,11 @@ def run_config(cx, rule, n, d, f, dtype, steps, warmup, want_e2e=False, e2e_step
     ms_step = float(ms_total.item()) / steps
     launches = nat.launch_count() - launches0
     nat.profile_enable(False)
+    if dump_dir:
+        cols, picks = last_step_outputs(cx, rule, G, out, d)
+        if rank == 0:
+            write_outputs(dump_dir, cols, picks)
+        del cols, picks
     # clocks under load: keep the same step loop running (untimed, same count on every rank) until two sampler periods
     # have passed since the timed region began
     need_ms = 2.2 * sampler.period_ms - float(ms_total.item())
@@ -624,7 +667,14 @@ def main():
                     help="append the C3/C4/C5 configurations (auto: only for the default headline workload)")
     ap.add_argument("--extra-steps", type=int, default=3)
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB; inputs are seeded, so "
+                         "two builds run with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps: at least one timed step")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm times a reduced CPU sample")
     if args.f is None:
         args.f = int(0.24 * args.n)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
@@ -654,7 +704,7 @@ def main():
     headline = (rule, n, d, args.dtype) == ("Krum", N_CLIENTS, DIM, "f32")
 
     rec = run_config(cx, rule, n, d, f, args.dtype, args.steps, args.warmup, want_e2e=True, e2e_steps=args.e2e_steps,
-                     check=not args.no_parity)
+                     check=not args.no_parity, dump_dir=args.dump_outputs)
     extras = []
     if args.extras == "on" or (args.extras == "auto" and headline):
         free_gb = torch.cuda.mem_get_info(device)[0] / 1e9

@@ -1,9 +1,12 @@
 """bench.py's reference arm (`--impl reference`) runs the CPU port of the reference algorithm and needs no
-GPU: check that it prints ONE JSON line with the contract's keys (tiny configuration, ~1 s of CPU work)."""
+GPU: check that it prints ONE JSON line with the contract's keys (tiny configuration, ~1 s of CPU work).
+`--dump-outputs`: the writer on CPU, the whole GPU arm on the device."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -108,3 +111,65 @@ while True:
     off = bench.ClockSampler(0)
     off.start(); off.align()
     assert off.stop()["sm_mhz"] is None
+
+
+def test_dump_outputs_files_and_sample(tmp_path):
+    """--dump-outputs: what the caller of each rule receives, float32 / float64 only; over the byte budget every vector is
+    cut to the same seeded column sample, identical from run to run."""
+    sys.path.insert(0, ROOT)
+    import bench
+    import numpy as np
+    import torch
+    from attacking_federate_learning_b200.sharded import ShardedAggregator
+
+    class Cx:
+        agg = ShardedAggregator()                   # one process: the vectors are already full length
+    G = torch.arange(5 * 1000, dtype=torch.float32).reshape(5, 1000)
+    cols, picks = bench.last_step_outputs(Cx, "Krum", G, 3, 1000)
+    bench.write_outputs(str(tmp_path / "krum"), cols, picks)
+    assert np.array_equal(np.load(tmp_path / "krum" / "aggregate.npy"), G[3].numpy())
+    idx = np.load(tmp_path / "krum" / "krum_index.npy")
+    assert idx.dtype == np.float64 and idx.tolist() == [3.0]
+    cols, picks = bench.last_step_outputs(Cx, "Bulyan", G, (G[1] + 0.5, torch.tensor([4, 0, 2], dtype=torch.int32)), 1000)
+    for run in ("b1", "b2"):
+        bench.write_outputs(str(tmp_path / run), cols, picks, budget=2000)
+        files = {p.name: np.load(p) for p in (tmp_path / run).iterdir()}
+        assert set(files) == {"aggregate.npy", "bulyan_selection.npy", "columns.npy"}
+        assert sum(p.stat().st_size for p in (tmp_path / run).iterdir()) <= 2000
+        assert all(a.dtype in (np.float32, np.float64) for a in files.values())
+        assert files["bulyan_selection.npy"].tolist() == [4.0, 0.0, 2.0]
+        pos = files["columns.npy"].astype(np.int64)
+        assert len(pos) > 50 and np.array_equal(files["aggregate.npy"], (G[1] + 0.5).numpy()[pos])
+    for name in ("aggregate.npy", "columns.npy"):
+        assert np.array_equal(np.load(tmp_path / "b1" / name), np.load(tmp_path / "b2" / name))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("rule", ["Krum", "Bulyan", "TrimmedMean", "ALIE"])
+def test_dump_outputs_of_the_timed_path(tmp_path, rule):
+    """Two runs with the same arguments write the same outputs; --steps is the number of timed steps."""
+    torch = pytest.importorskip("torch")
+    if not torch.cuda.is_available():
+        pytest.skip("no GPU")
+    import numpy as np
+    n, d, f = 23, 40000, 5
+    outs = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--rule", rule, "--n", str(n), "--d", str(d),
+                              "--f", str(f), "--steps", "4", "--warmup", "3", "--no-cpu-baseline", "--e2e-steps", "0",
+                              "--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=600, cwd=ROOT,
+                             env=dict(os.environ, AFL_BENCH_CLOCKS_MS="0"))
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][0])
+        assert line["steps"] == 4 and line["parity"]["match"]
+        outs.append({p.name: np.load(p) for p in (tmp_path / run).iterdir()})
+    a, b = outs
+    assert set(a) == set(b) and all(np.array_equal(a[k], b[k]) for k in a)
+    vec = a.pop("crafted.npy" if rule == "ALIE" else "aggregate.npy")
+    assert vec.dtype == np.float32 and vec.shape == (d,) and np.isfinite(vec).all()
+    want = {"Krum": {"krum_index.npy"}, "Bulyan": {"bulyan_selection.npy"}}.get(rule, set())
+    assert set(a) == want and all(v.dtype == np.float64 for v in a.values())
+    if rule == "Krum":
+        assert 0 <= a["krum_index.npy"][0] < n
+    if rule == "Bulyan":
+        assert len(a["bulyan_selection.npy"]) == n - 2 * f

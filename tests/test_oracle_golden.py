@@ -1,17 +1,13 @@
-"""Pin oracle/ref_numpy.py to outputs of the unmodified reference (tests/golden/golden_v1.npz,
-generated by tests/golden/make_golden.py) — bit for bit — and, in the build container where
-/root/reference exists, to the live reference on fresh random inputs."""
+"""Pin oracle/ref_numpy.py to outputs of the unmodified reference — bit for bit: the edge cases and
+shapes of tests/golden/golden_v1.npz (tests/golden/make_golden.py) and the seeded random cases of
+tests/golden/golden_seeded_v1.npz (tests/golden/make_golden_seeded.py)."""
 import os
-import sys
 
 import numpy as np
 import pytest
 
-from conftest import golden_names
+from conftest import ROOT, golden_names
 from oracle import ref_numpy as orc
-
-REF_DIR = os.environ.get("AFL_REFERENCE_DIR", "/root/reference")
-HAVE_REF = os.path.exists(os.path.join(REF_DIR, "defences.py"))
 
 
 def same_bits(a, b):
@@ -109,26 +105,21 @@ def test_edge_semantics(golden):
     # answer is not a function of the values alone -> documented as undefined, not pinned.
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="live reference only exists in the build container")
-@pytest.mark.parametrize("seed", range(6))
-def test_against_live_reference(seed):
-    sys.path.insert(0, REF_DIR)
-    import defences as ref_def
-    import malicious as ref_mal
-    rng = np.random.default_rng(1000 + seed)
-    n = int(rng.integers(3, 40)); d = int(rng.integers(1, 300)); f = int(rng.integers(0, max(1, (n - 3) // 4 + 1)))
-    G = (0.1 * rng.standard_normal(d) + np.exp(0.25 * rng.standard_normal((n, 1))) * rng.standard_normal((n, d))).astype(np.float32)
-    if seed % 2:
-        G[:max(f, 2)] = G[0]                                            # identical rows
-    assert orc.krum(G, n, f, return_index=True) == ref_def.krum(G, n, f, return_index=True)
-    assert same_bits(orc.trimmed_mean(G, n, f), ref_def.trimmed_mean(G, n, f))
-    assert same_bits(orc.no_defense(G), ref_def.no_defense(G, n, f))
-    if n >= 4 * f + 3:
-        assert same_bits(orc.bulyan(G, n, f), ref_def.bulyan(G, n, f))
+@pytest.fixture(scope="module")
+def golden_seeded():
+    return np.load(os.path.join(ROOT, "tests", "golden", "golden_seeded_v1.npz"), allow_pickle=False)
 
-    class U:  # duck-typed user, as malicious.py expects
-        def __init__(self, g): self.grads = g; self.original_params = None; self.learning_rate = None
-    users = [U(G[i].copy()) for i in range(max(f, 1))]
-    att = ref_mal.DriftAttack(1.5); att.attack(users)
-    crafted, mu, sigma = orc.alie_attack([G[i].copy() for i in range(max(f, 1))], 1.5)
-    assert same_bits(crafted, users[0].grads) and same_bits(sigma, att.grads_stdev)
+
+@pytest.mark.parametrize("seed", range(6))
+def test_against_live_reference(golden_seeded, seed):
+    """Random N, D, f (identical leading rows for odd seeds): every rule and the ALIE attack against what the
+    reference returned on the same matrix."""
+    g = {k.split("/", 1)[1]: golden_seeded[k] for k in golden_seeded.files if k.startswith(f"seed{seed}/")}
+    G, f = g["G"], int(g["f"]); n = len(G)
+    assert orc.krum(G, n, f, return_index=True) == int(g["krum_idx"])
+    assert same_bits(orc.trimmed_mean(G, n, f), g["tm"])
+    assert same_bits(orc.no_defense(G), g["mean"])
+    if n >= 4 * f + 3:
+        assert same_bits(orc.bulyan(G, n, f), g["bulyan"])
+    crafted, mu, sigma = orc.alie_attack([G[i].copy() for i in range(max(f, 1))], float(g["alie_z"]))
+    assert same_bits(crafted, g["alie_grads0"]) and same_bits(sigma, g["alie_stdev"])
