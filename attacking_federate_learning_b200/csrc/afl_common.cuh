@@ -50,8 +50,8 @@ static inline cudaError_t ensure_dyn_smem(K kernel, int bytes, int (&done)[kMaxD
   return e;
 }
 
-// Optional tail of the split reduction (csrc/xgpu.cu): the LAST block to finish also forms the squared-distance
-// table and publishes this rank's epoch flag to every peer, which saves two launches per multi-GPU Krum step.
+// Optional tail of gram_to_sqdist_kernel (csrc/xgpu.cu): the LAST block to finish also publishes this rank's epoch
+// flag to every peer, which saves a launch per multi-GPU Krum step.
 constexpr int kMaxWorld = 16;
 struct PubHook {
   unsigned long long* flag[kMaxWorld];   // flags block of every rank (peer-mapped)
@@ -286,6 +286,94 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
 // [7,10) | b_format TF32 (2) [10,13) | a/b K-major (0) | n>>3 [17,23) | m>>4 [24,29).
 __host__ __device__ __forceinline__ uint32_t umma_idesc_tf32(uint32_t m, uint32_t n) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+// c_format F32 (1) [4,6) | a_format BF16 (1) [7,10) | b_format BF16 (1) [10,13) | K-major | n>>3 | m>>4
+__host__ __device__ __forceinline__ uint32_t umma_idesc_bf16(uint32_t m, uint32_t n) {
+  return (1u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+// K-major, SWIZZLE_128B, 128-byte rows, 8-row groups `sbo` bytes apart.
+__device__ __forceinline__ uint64_t umma_desc_sw128_sbo(uint32_t smem_addr, uint32_t sbo) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr & 0x3FFFFu) >> 4);
+  d |= static_cast<uint64_t>(1) << 16;
+  d |= static_cast<uint64_t>(sbo >> 4) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(2) << 61;
+  return d;
+}
+// D[tmem] (+)= A[smem desc] * B[smem desc]^T, BF16 inputs, fp32 accumulate, issued by ONE thread.
+__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
+      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// 32 lanes x 8 consecutive fp32 columns -> 8 registers per thread.
+__device__ __forceinline__ void tmem_ld_32x32b_x8(uint32_t taddr, uint32_t (&v)[8]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
+               : "r"(taddr) : "memory");
+}
+
+// ------------------------------------------------------------------------------------------------
+// bf16x2 operands, converted in place (gram_bf16.cu, gram_pair.cu)
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t pack_bf16x2_rn(float lo, float hi) {
+  uint32_t r;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+__device__ __forceinline__ void sts64(uint32_t addr, uint32_t a, uint32_t b) {
+  asm volatile("st.shared.v2.b32 [%0], {%1,%2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
+}
+// Per-lane constants of bf16x2_convert_units: a half warp owns one 256-byte fp32 row (16 lanes x 16 bytes), the warp
+// reads 2 rows per LDS.128 and an 8-row unit (2 KB) with 4 of them.  The lane with fp32 chunk c16 owns bf16 bytes
+// [8 c16, 8 c16 + 8) of the 128-byte bf16 row, i.e. half of 16-byte chunk c16/2, which SWIZZLE_128B places at chunk
+// (c16/2) ^ (row & 7).  dst_off[u]: destination of row 2u + rsub inside the unit's atom.
+__device__ __forceinline__ void bf16x2_lane_offsets(uint32_t& src_lane, uint32_t (&dst_off)[4]) {
+  const int rsub = lane_id() >> 4, c16 = lane_id() & 15;
+#pragma unroll
+  for (int u = 0; u < 4; ++u) {
+    const uint32_t row8 = static_cast<uint32_t>(2 * u + rsub);
+    dst_off[u] = row8 * 128u + ((static_cast<uint32_t>(c16 >> 1) ^ row8) << 4) + (static_cast<uint32_t>(c16 & 1) << 3);
+  }
+  src_lane = static_cast<uint32_t>(rsub) * 256u + static_cast<uint32_t>(c16) * 16u;
+}
+// Rewrites `units` 8-row units of fp32 (2 KB each, 256-byte rows of 64 columns, from `base`) IN PLACE: unit u
+// becomes one SWIZZLE_128B core-matrix atom of b1 at base + 2048 u followed by one of b2 at base + 2048 u + 1024,
+// with g - c = b1 + b2 + r, |r| <= 2^-17 |g - c| (both roundings to nearest); c = this lane's 4 columns of the
+// centre.  A unit's output only overwrites that unit's own input, which the warp has already loaded.
+__device__ __forceinline__ void bf16x2_convert_units(uint32_t base, int units, uint32_t src_lane,
+                                                     const uint32_t (&dst_off)[4], float4 cen) {
+  float4 v[4];
+#pragma unroll
+  for (int u = 0; u < 4; ++u) v[u] = lds128(base + src_lane + static_cast<uint32_t>(u) * 512u);
+#pragma unroll 1
+  for (int unit = 0; unit < units; ++unit) {
+    uint32_t h[4][2], l[4][2];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const float x0 = v[u].x - cen.x, x1 = v[u].y - cen.y, x2 = v[u].z - cen.z, x3 = v[u].w - cen.w;
+      h[u][0] = pack_bf16x2_rn(x0, x1);
+      h[u][1] = pack_bf16x2_rn(x2, x3);
+      l[u][0] = pack_bf16x2_rn(x0 - __uint_as_float(h[u][0] << 16), x1 - __uint_as_float(h[u][0] & 0xFFFF0000u));
+      l[u][1] = pack_bf16x2_rn(x2 - __uint_as_float(h[u][1] << 16), x3 - __uint_as_float(h[u][1] & 0xFFFF0000u));
+    }
+    const uint32_t ub = base + static_cast<uint32_t>(unit) * 2048u;
+    if (unit + 1 < units) {                               // next unit's loads before this unit's stores
+#pragma unroll
+      for (int u = 0; u < 4; ++u) v[u] = lds128(ub + 2048u + src_lane + static_cast<uint32_t>(u) * 512u);
+    }
+    __syncwarp();                                         // every lane has read this unit before anyone overwrites it
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      sts64(ub + dst_off[u], h[u][0], h[u][1]);
+      sts64(ub + 1024u + dst_off[u], l[u][0], l[u][1]);
+    }
+  }
 }
 
 // Centre of the bf16x2 Gram kernels: mean of the LAST `rows` clients (cref = first of those rows, pitch ld) over

@@ -362,78 +362,39 @@ gram_reduce_kernel(const float* __restrict__ parts, int n, int tiles, int splits
   }
 }
 
-// gram_reduce_kernel + gram_to_sqdist_kernel (+ the publish of csrc/xgpu.cu) in one launch, single-tile tables only:
-// every block reduces its row as above; the last block to finish (atomic counter) forms d2 and stores the epoch flag
-// into every peer's flag block.
-__global__ void __launch_bounds__(128 * kSy)
-gram_reduce_d2_kernel(const float* __restrict__ parts, int n, int splits, double* HX, double* __restrict__ d2, const PubHook hook) {
-  __shared__ double sh[kSy][128];
-  __shared__ int s_last;
-  const int i = blockIdx.x, a = blockIdx.y;
-  const int jj = threadIdx.x, sy = threadIdx.y;
-  const float* base = parts + static_cast<size_t>(a) * kTileRows * kTileRows + i * kTileRows + jj;
-  const int s0 = splits * sy / kSy, s1 = splits * (sy + 1) / kSy;
-  double acc = 0.0;
-  if (jj < n)
-    for (int s = s0; s < s1; ++s) acc += static_cast<double>(base[static_cast<size_t>(s) * kPartElems]);
-  sh[sy][jj] = acc;
-  __syncthreads();
-  if (sy == 0 && jj < n) {
-    double t = sh[0][jj];
-#pragma unroll
-    for (int y = 1; y < kSy; ++y) t += sh[y][jj];
-    HX[(static_cast<size_t>(a) * n + i) * n + jj] = t;
-  }
-  __threadfence();
-  __syncthreads();
-  const int tid = threadIdx.y * 128 + threadIdx.x;
-  if (tid == 0) s_last = (atomicAdd(hook.counter, 1u) == gridDim.x * gridDim.y - 1u) ? 1 : 0;
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  const double* H = HX;
-  const double* X = HX + static_cast<size_t>(n) * n;
-  for (int e = tid; e < n * n; e += 128 * kSy) {
-    const int r = e / n, c = e - r * n;
-    double v = 0.0;
-    if (r != c) {
-      const int lo = min(r, c), hi = max(r, c);
-      const size_t ll = static_cast<size_t>(lo) * n + lo, hh = static_cast<size_t>(hi) * n + hi;
-      const size_t lh = static_cast<size_t>(lo) * n + hi, hl = static_cast<size_t>(hi) * n + lo;
-      const double s_ll = __ldcg(H + ll) + (__ldcg(X + ll) + __ldcg(X + ll));
-      const double s_hh = __ldcg(H + hh) + (__ldcg(X + hh) + __ldcg(X + hh));
-      const double s_lh = __ldcg(H + lh) + (__ldcg(X + lh) + __ldcg(X + hl));
-      v = (s_ll + s_hh) - 2.0 * s_lh;
-    }
-    d2[e] = v;
-  }
-  __syncthreads();
-  if (tid == 0) *hook.counter = 0u;
-  if (hook.world > 1 && tid < hook.world) {
-    __threadfence_system();
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(hook.flag[tid] + hook.rank), "l"(hook.epoch) : "memory");
-  }
-}
-
 // d2_ij = s_ii + s_jj - 2 s_ij with s_ij = hh_ij + (x_ij + x_ji); x_ij + x_ji is commutative, so s (and d2)
-// are exactly symmetric, and identical rows give exact zeros.
-__global__ void gram_to_sqdist_kernel(const double* __restrict__ HX, int n, double* __restrict__ d2) {
+// are exactly symmetric, and identical rows give exact zeros.  hook.counter != null: the last block to finish also
+// publishes this rank's epoch flag to every peer (csrc/xgpu.cu), which saves a launch per multi-GPU Krum step.
+__global__ void gram_to_sqdist_kernel(const double* __restrict__ HX, int n, double* __restrict__ d2, const PubHook hook) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   const int i = blockIdx.y;
-  if (j >= n) return;
-  const double* H = HX;
-  const double* X = HX + static_cast<size_t>(n) * n;
-  double v = 0.0;
-  if (i != j) {
-    const int lo = min(i, j), hi = max(i, j);
-    const size_t ll = static_cast<size_t>(lo) * n + lo, hh = static_cast<size_t>(hi) * n + hi;
-    const size_t lh = static_cast<size_t>(lo) * n + hi, hl = static_cast<size_t>(hi) * n + lo;
-    const double s_ll = H[ll] + (X[ll] + X[ll]);
-    const double s_hh = H[hh] + (X[hh] + X[hh]);
-    const double s_lh = H[lh] + (X[lh] + X[hl]);
-    v = (s_ll + s_hh) - 2.0 * s_lh;
+  if (j < n) {
+    const double* H = HX;
+    const double* X = HX + static_cast<size_t>(n) * n;
+    double v = 0.0;
+    if (i != j) {
+      const int lo = min(i, j), hi = max(i, j);
+      const size_t ll = static_cast<size_t>(lo) * n + lo, hh = static_cast<size_t>(hi) * n + hi;
+      const size_t lh = static_cast<size_t>(lo) * n + hi, hl = static_cast<size_t>(hi) * n + lo;
+      const double s_ll = H[ll] + (X[ll] + X[ll]);
+      const double s_hh = H[hh] + (X[hh] + X[hh]);
+      const double s_lh = H[lh] + (X[lh] + X[hl]);
+      v = (s_ll + s_hh) - 2.0 * s_lh;
+    }
+    d2[static_cast<size_t>(i) * n + j] = v;
   }
-  d2[static_cast<size_t>(i) * n + j] = v;
+  if (!hook.counter) return;
+  __shared__ int s_last;
+  __threadfence_system();                                  // this block's rows, before its count
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = (atomicAdd(hook.counter, 1u) == gridDim.x * gridDim.y - 1u) ? 1 : 0;
+  __syncthreads();
+  if (!s_last) return;
+  if (threadIdx.x == 0) *hook.counter = 0u;
+  if (threadIdx.x < hook.world) {
+    __threadfence_system();
+    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(hook.flag[threadIdx.x] + hook.rank), "l"(hook.epoch) : "memory");
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -653,7 +614,7 @@ int sqdist_partial(const void* G, int n, int64_t d, int64_t ld, int dtype, doubl
   return sqdist_partial_ex(G, n, d, ld, dtype, d2_out, ws, ws_bytes, flags, stream, nullptr, nullptr);
 }
 // hook != null: the caller (csrc/xgpu.cu) wants its epoch flag published once d2_out is complete; *hook_done tells
-// whether the reduction kernel did it (single-tile bf16x2 path) or the caller still has to launch its publish kernel.
+// whether gram_to_sqdist_kernel did it (single-tile bf16x2 path) or the caller still has to launch its publish kernel.
 int sqdist_partial_ex(const void* G, int n, int64_t d, int64_t ld, int dtype, double* d2_out, void* ws, size_t ws_bytes,
                       int flags, cudaStream_t stream, const PubHook* hook, bool* hook_done) {
   if (hook_done) *hook_done = false;
@@ -683,16 +644,14 @@ int sqdist_partial_ex(const void* G, int n, int64_t d, int64_t ld, int dtype, do
       double* S = reinterpret_cast<double*>(static_cast<uint8_t*>(ws) + pl.parts_bytes);
       int rc = launch_bf16x2(static_cast<const float*>(G), n, d, ld, parts, pl.splits, pl.flush, center, stream);
       if (rc) return rc;
-      if (hook && hook->counter) {
-        gram_reduce_d2_kernel<<<dim3(n, 2, 1), dim3(128, kSy), 0, stream>>>(parts, n, pl.splits, S, d2_out, *hook);
-        AFL_LAUNCH_CHECK("gram_reduce_d2_kernel");
-        if (hook_done) *hook_done = true;
-        return AFL_OK;
-      }
       gram_reduce_kernel<<<dim3(n, 2, 1), dim3(128, kSy), 0, stream>>>(parts, n, 1, pl.splits, S);
       AFL_LAUNCH_CHECK("gram_reduce_kernel");
-      gram_to_sqdist_kernel<<<rgrid, rblock, 0, stream>>>(S, n, d2_out);
+      const bool pub = hook && hook->counter;
+      PubHook h{};
+      if (pub && hook->world > 1) h = *hook;           // a single rank has no flag to publish
+      gram_to_sqdist_kernel<<<rgrid, rblock, 0, stream>>>(S, n, d2_out, h);
       AFL_LAUNCH_CHECK("gram_to_sqdist_kernel");
+      if (hook_done) *hook_done = pub;
       return AFL_OK;
     }
     EncodeTiledFn enc = encode_fn();
@@ -752,7 +711,7 @@ int sqdist_partial_ex(const void* G, int n, int64_t d, int64_t ld, int dtype, do
     AFL_LAUNCH_CHECK("gram_tcgen05_kernel");
     gram_reduce_kernel<<<dim3(n, 2, pl.tiles), dim3(128, kSy), 0, stream>>>(p.parts, n, pl.tiles, pl.splits, S);
     AFL_LAUNCH_CHECK("gram_reduce_kernel");
-    gram_to_sqdist_kernel<<<rgrid, rblock, 0, stream>>>(S, n, d2_out);
+    gram_to_sqdist_kernel<<<rgrid, rblock, 0, stream>>>(S, n, d2_out, PubHook{});
     AFL_LAUNCH_CHECK("gram_to_sqdist_kernel");
   } else {
     const int t32 = (n + 31) / 32;

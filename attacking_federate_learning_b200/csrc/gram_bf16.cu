@@ -6,35 +6,40 @@
 // gram.cu needs >= 620 tensor cycles per 32 columns, more than the ~550 cycles HBM needs for them, while
 // bf16 operands need 310.  Here:
 //
-//   * TMA (cp.async.bulk.tensor.2d, no swizzle, zero OOB fill) streams one k-block [N x 64] of fp32 per
-//     instruction into a 4-slot ring.  tools/tma_bench.cu measured a fixed ~450 ns per 2-D box per SM
-//     whatever its size (25..100 rows, 128..512 B rows), so 128-byte-wide boxes cap at 3.8 TB/s chip-wide
-//     while 256-byte-wide boxes reach the HBM bound; the raw layout is free because only the converters
-//     read it;
-//   * 4 converter warps (one per ring slot / operand stage) turn the fp32 k-block into one bf16 operand
-//     stage: every value is split into two bf16 terms, g = b1 + b2 + r (both roundings to nearest,
-//     |r| <= 2^-17 |g|), stored as b1 || b2, K-major, 64 columns per 128-byte row, SWIZZLE_128B.  A half
-//     warp reads one 256-byte fp32 row and writes one 128-byte bf16 row of b1 and of b2 (conflict-free);
-//   * S ~= b1 b1^T + b1 b2^T + (b1 b2^T)^T: ONE tcgen05.mma.kind::f16 (K = 16) per 16 columns with
-//     A = b1 (M = 128) and B = b1 || b2 (N = 2*N_pad), fp32 accumulation in TMEM.  Dropped terms
-//     (b2 b2^T, r) are ~2^-17 relative per product; b2 b2^T is positive on every squared distance and
-//     shows up as a uniform ~-1.3e-6 scale of d2;
-//   * two MMA issuer warps alternate k-blocks, TMEM accumulators are double-buffered and drained every
-//     `flush` k-blocks by 8 epilogue warps into fp32 registers, K is interleaved over the CTAs into
-//     private partial slots that gram_reduce_kernel sums in a fixed order in float64 (bit-reproducible;
-//     identical rows give exact zeros and identical table rows).
+//   * TMA (cp.async.bulk.tensor.2d, no swizzle, zero OOB fill) streams one k-block {64 fp32 columns x N_pad
+//     rows} per instruction into a 7-slot ring (slot = k-block % 7; rows N..N_pad-1 are zero fill).
+//     tools/tma_bench.cu measured a fixed ~450 ns per 2-D box per SM whatever its size, so 128-byte-wide
+//     boxes cap at 3.8 TB/s chip-wide while 256-byte-wide boxes reach the HBM bound;
+//   * 4 converter warps (warp w takes k-blocks w, w+4, ...) rewrite the slot IN PLACE
+//     (bf16x2_convert_units, shared with gram_pair.cu): every 8-row unit u (2 KB of fp32) becomes one
+//     SWIZZLE_128B core-matrix atom of b1 at slot + 2048 u followed by one of b2 at slot + 2048 u + 1024,
+//     g - c = b1 + b2 + r (both roundings to nearest, |r| <= 2^-17 |g - c|), c = the mean of the last 8
+//     clients' rows of the same k-block, read from the slot before its first store.  Without a second
+//     staging buffer the ring holds 7 k-blocks in flight instead of 4: a slot lives for TMA latency +
+//     conversion + MMA, and the ring depth, not HBM, paced the 4-slot version (Little's law);
+//   * S ~= b1 b1^T + b1 b2^T + (b1 b2^T)^T: ONE tcgen05.mma.kind::f16 (K = 16) per 16 columns.  A = b1
+//     (M = 128, 8-row groups 2048 bytes apart from the slot base; rows >= N_pad reach past the slot and
+//     land in result rows nobody reads) and B = the whole slot with 8-row groups 1024 bytes apart, i.e.
+//     N = 2*N_pad rows b1 unit 0, b2 unit 0, b1 unit 1, ...: result column 16 u + r holds b1 b1^T of client
+//     8 u + r, column 16 u + 8 + r holds b1 b2^T.  Dropped terms (b2 b2^T, r) are ~2^-17 relative per
+//     product; b2 b2^T is positive on every squared distance and shows up as a uniform ~-1.3e-6 scale of d2;
+//   * the MMA commit of a k-block returns its slot to the TMA producer.  Two MMA issuer warps alternate
+//     k-blocks strictly (named barriers 8 and 9), so every CTA accumulates in k-block order; TMEM
+//     accumulators are double-buffered and drained every `flush` k-blocks by 8 epilogue warps into fp32
+//     registers, K is interleaved over the CTAs into private partial slots that gram_reduce_kernel sums in a
+//     fixed order in float64 (bit-reproducible; identical rows give exact zeros and identical table rows).
 //
 // Warp roles (512 threads): warp 0 TMA producer, warps 1,3 MMA issue, warp 2 TMEM alloc, warps 4-7
-// converters, warps 8-15 epilogue.
+// converters, warps 8-15 epilogue (warp group a drains the 8-column groups 2u + a).
 #include "afl_common.cuh"
 
 namespace afl {
 namespace gram {
 
 constexpr int kB16Threads = 512;
-constexpr int kRawSlots = 4;         // fp32 k-blocks [n x 64 cols] in the TMA ring (slot = k-block % 4)
-constexpr int kBfStages = 4;         // bf16 operand stages [2*nb rows x 64 cols]
+constexpr int kB16Slots = 7;         // ring slots, one k-block [N_pad x 64 fp32] each (slot = k-block % 7)
 constexpr int kB16Cols = 64;         // fp32 columns per k-block = 128 bytes of bf16 per row
+constexpr int kB16ASpan = 16 * 2048; // bytes the A operand (128 rows, 2 KB per 8-row group) spans from its slot base
 constexpr int kB16PartElems = 2 * 128 * 128;
 
 struct B16Params {
@@ -43,57 +48,25 @@ struct B16Params {
   int kblocks;          // ceil(d / 64)
   int flush;            // k-blocks per TMEM accumulation chain (even)
   float* parts;         // [splits][2][128][128]
-  int center;           // subtract the last client's row while converting (translation invariance)
-  const float* cref;    // first of the last cref_rows rows
-  int cref_rows; int64_t cref_ld;
-  int64_t d;
+  int center;           // subtract the mean of the last clients' rows while converting (translation invariance)
 };
-
-__device__ __forceinline__ uint32_t pack_bf16x2_rn(float lo, float hi) {
-  uint32_t r;
-  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-  return r;
-}
-__device__ __forceinline__ void sts128_u(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ void sts64_u(uint32_t addr, uint32_t a, uint32_t b) {
-  asm volatile("st.shared.v2.b32 [%0], {%1,%2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                          uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// c_format F32 (1) [4,6) | a_format BF16 (1) [7,10) | b_format BF16 (1) [10,13) | K-major | n>>3 | m>>4
-__host__ __device__ __forceinline__ uint32_t umma_idesc_bf16(uint32_t m, uint32_t n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
-}
 
 __global__ void __launch_bounds__(kB16Threads, 1)
 gram_bf16x2_kernel(const __grid_constant__ CUtensorMap tmap, const B16Params p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  __shared__ __align__(8) uint64_t raw_full[kRawSlots], raw_empty[kRawSlots], bf_empty[kBfStages], acc_full[2],
-      acc_empty[2], first_issued[2];
+  __shared__ __align__(8) uint64_t raw_full[kB16Slots], slot_free[kB16Slots], acc_full[2], acc_empty[2], first_issued[2];
   __shared__ uint32_t tmem_base_smem;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wg = warp >> 2;
   const int split = blockIdx.x;
   const int nkb = (p.kblocks - split + p.splits - 1) / p.splits;      // k-blocks split, split+splits, ...
   const int ngroups = (nkb + p.flush - 1) / p.flush;
-  const uint32_t raw_bytes = static_cast<uint32_t>(p.n) * 256u;       // one fp32 k-block [n x 64], row-major
-  const uint32_t stage_bytes = static_cast<uint32_t>(p.nb) * 256u;    // b1 (nb rows) || b2 (nb rows)
-  const uint32_t raw_base = smem_u32(smem);
-  const uint32_t bf_base = (raw_base + kRawSlots * raw_bytes + 1023u) & ~1023u;
+  const uint32_t slot_bytes = static_cast<uint32_t>(p.nb) * 256u;     // one fp32 k-block [nb x 64], row-major
+  const uint32_t ring = smem_u32(smem);
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < kRawSlots; ++s) { mbar_init(&raw_full[s], 1); mbar_init(&raw_empty[s], 1); }
-    for (int s = 0; s < kBfStages; ++s) mbar_init(&bf_empty[s], 1);
+    for (int s = 0; s < kB16Slots; ++s) { mbar_init(&raw_full[s], 1); mbar_init(&slot_free[s], 1); }
     for (int b = 0; b < 2; ++b) {
       mbar_init(&acc_full[b], 2);
       mbar_init(&acc_empty[b], 8);
@@ -109,28 +82,28 @@ gram_bf16x2_kernel(const __grid_constant__ CUtensorMap tmap, const B16Params p) 
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  const uint32_t tmem_base = tmem_base_smem;
+  // tmem_base_smem is read where it is used: kept live through the converters' 112 registers it would spill
 
   if (wg == 0) {
     setmaxnreg_dec<64>();
     if (warp == 0) {
-      // ===================== TMA producer: one box [n x 64 fp32] per k-block =====================
+      // ===================== TMA producer: one box [nb x 64 fp32] per k-block =====================
       if (lane == 0) {
         const uint64_t pol = policy_evict_first();
         int s = 0;
         uint32_t ph = 0;
         for (int i = 0; i < nkb; ++i) {
-          mbar_wait(&raw_empty[s], ph ^ 1);
-          mbar_arrive_expect_tx(&raw_full[s], raw_bytes);
-          tma_load_2d(smem + static_cast<size_t>(s) * raw_bytes, &tmap, &raw_full[s], (split + i * p.splits) * kB16Cols, 0, pol);
-          if (++s == kRawSlots) { s = 0; ph ^= 1; }
+          mbar_wait(&slot_free[s], ph ^ 1);
+          mbar_arrive_expect_tx(&raw_full[s], slot_bytes);
+          tma_load_2d(smem + static_cast<size_t>(s) * slot_bytes, &tmap, &raw_full[s], (split + i * p.splits) * kB16Cols, 0, pol);
+          if (++s == kB16Slots) { s = 0; ph ^= 1; }
         }
       }
     } else if (warp == 1 || warp == 3) {
       // ===================== MMA issuers (alternating k-blocks) =====================
       const int j = (warp == 3) ? 1 : 0;
       const uint32_t idesc = umma_idesc_bf16(128, 2 * p.nb);
-      int s = j;
+      const uint32_t tmem_base = tmem_base_smem;
       for (int g = 0; g < ngroups; ++g) {
         const int b = g & 1;
         const uint32_t gph = (g >> 1) & 1;
@@ -143,20 +116,25 @@ gram_bf16x2_kernel(const __grid_constant__ CUtensorMap tmap, const B16Params p) 
         else mbar_wait_fast(&first_issued[b], gph);
         tc_fence_after();
         for (; it < it_end; it += 2) {
-          named_bar_sync(1 + s, 32 + 32);                // converter warp s has written and fenced stage s
+          const int s = it % kB16Slots;
+          named_bar_sync(1 + s, 32 + 32);                // the converter warp of k-block `it` has written and fenced slot s
+          // Strict alternation: k-block `it` is issued only after k-block it-1 has been, so the accumulation order is
+          // the k-block order (reproducible run to run).  Barrier 8: issuer 0 -> 1, barrier 9: issuer 1 -> 0.
+          if (it > 0) named_bar_sync(j == 0 ? 9u : 8u, 32 + 32);
           tc_fence_after();
-          const uint64_t dab = umma_desc_sw128(bf_base + static_cast<uint32_t>(s) * stage_bytes);
-          if (elect_one()) {                             // A = rows 0..127 of the stage, B = rows 0..2nb-1
+          const uint32_t slot = ring + static_cast<uint32_t>(s) * slot_bytes;
+          const uint64_t da = umma_desc_sw128_sbo(slot, 2048u);   // A = b1 atoms: rows 0..127
+          const uint64_t db = umma_desc_sw128_sbo(slot, 1024u);   // B = b1, b2 atoms alternating: rows 0..2nb-1
+          if (elect_one()) {
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks)               // 4 x K=16 bf16 = 64 columns; +32 bytes per step
-              umma_bf16(d_acc, dab + static_cast<uint64_t>(ks * 2), dab + static_cast<uint64_t>(ks * 2), idesc,
+              umma_bf16(d_acc, da + static_cast<uint64_t>(ks * 2), db + static_cast<uint64_t>(ks * 2), idesc,
                         (it != it_begin) || (ks != 0));
-            umma_commit(&bf_empty[s]);
+            umma_commit(&slot_free[s]);
             if (it == it_begin) mbar_arrive(&first_issued[b]);
           }
           __syncwarp();
-          s += 2;
-          if (s >= kBfStages) s -= kBfStages;
+          if (it + 1 < nkb) named_bar_arrive(j == 0 ? 8u : 9u, 32 + 32);
         }
         if (elect_one()) umma_commit(&acc_full[b]);
         __syncwarp();
@@ -164,106 +142,46 @@ gram_bf16x2_kernel(const __grid_constant__ CUtensorMap tmap, const B16Params p) 
     }
   } else if (wg == 1) {
     setmaxnreg_dec<112>();
-    // ===================== converters: one fp32 k-block -> one bf16 stage b1 || b2 =====================
-    // Converter warp w owns ring slot w, operand stage w and k-blocks w, w+4, ...: four k-blocks are
-    // converted in parallel.  A half warp takes one fp32 row (16 lanes x 16 bytes = 64 columns): the lane
-    // with fp32 chunk c16 owns bf16 bytes [8*c16, 8*c16+8) of the 128-byte bf16 row, i.e. half of the
-    // 16-byte chunk c16/2, which SWIZZLE_128B places at chunk (c16/2) ^ (row & 7).
+    // ===================== converters: fp32 k-block -> b1 / b2 atoms, in place =====================
     const int w4 = warp - 4;
-    const uint32_t src = raw_base + static_cast<uint32_t>(w4) * raw_bytes;
-    const uint32_t dst = bf_base + static_cast<uint32_t>(w4) * stage_bytes;
-    const uint32_t dst2 = dst + static_cast<uint32_t>(p.nb) * 128u;
-    for (int i = lane; i < (p.nb - p.n) * 8; i += 32) {   // pad rows n..nb-1 stay zero for the whole kernel
-      const uint32_t off = static_cast<uint32_t>(p.n) * 128u + static_cast<uint32_t>(i) * 16u;
-      sts128_u(dst + off, 0u, 0u, 0u, 0u);
-      sts128_u(dst2 + off, 0u, 0u, 0u, 0u);
-    }
-    const int rsub = lane >> 4, c16 = lane & 15;
-    const uint32_t src_lane = src + static_cast<uint32_t>(rsub) * 256u + static_cast<uint32_t>(c16) * 16u;
-    // Row r0 + 2u + rsub (r0 a multiple of 16): the swizzle term only depends on (2u + rsub) & 7, so the
-    // destination offset is r0*128 + u*256 + one of four per-lane constants.
-    uint32_t lane_off[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-      lane_off[k] = static_cast<uint32_t>(rsub) * 128u + (static_cast<uint32_t>(c16 & 1) << 3) +
-                    (static_cast<uint32_t>((c16 >> 1) ^ ((2 * k + rsub) & 7)) << 4);
-    const int full_rows = p.n & ~15;
+    uint32_t src_lane, dst_off[4];
+    bf16x2_lane_offsets(src_lane, dst_off);
+    const int units = p.nb >> 3;
     // centre = mean of the last 8 clients over this lane's 4 columns; their rows are part of the k-block that TMA
     // just delivered, so they are read from shared memory (8 broadcast LDS.128 per k-block) - no extra L2 traffic
     const int crow0 = p.n >= kGramCenterRows ? p.n - kGramCenterRows : 0;
-    const uint32_t cen_off = static_cast<uint32_t>(c16) * 16u;
-    for (int kb = w4; kb < nkb; kb += kBfStages) {
-      const uint32_t ph = static_cast<uint32_t>(kb / kBfStages) & 1u;
-      mbar_wait_fast(&bf_empty[w4], ph ^ 1);
-      mbar_wait_fast(&raw_full[w4], ph);
+    const uint32_t cen_off = static_cast<uint32_t>(lane & 15) * 16u;
+    for (int kb = w4; kb < nkb; kb += 4) {
+      const int s = kb % kB16Slots;
+      const uint32_t ph = static_cast<uint32_t>(kb / kB16Slots) & 1u;
+      // k-block kb - 7 (another converter's) may still be in flight: the copies of two TMA boxes complete in no
+      // defined order, and while raw_full[s] is still in kb - 7's phase a wait for kb's parity would see the phase
+      // before it as complete.  kb - 7's MMA commit (the producer's own wait before loading kb) closes that window.
+      if (kb >= kB16Slots) mbar_wait_fast(&slot_free[s], ph ^ 1u);
+      mbar_wait_fast(&raw_full[s], ph);
+      const uint32_t slot = ring + static_cast<uint32_t>(s) * slot_bytes;
       float4 cen = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (p.center) {
+      if (p.center) {                                     // before the first store: the last rows are overwritten last
         float4 t[kGramCenterRows];
 #pragma unroll
         for (int r = 0; r < kGramCenterRows; ++r) {
           const int row = crow0 + r < p.n ? crow0 + r : p.n - 1;
-          t[r] = lds128(src + static_cast<uint32_t>(row) * 256u + cen_off);
+          t[r] = lds128(slot + static_cast<uint32_t>(row) * 256u + cen_off);
         }
 #pragma unroll
         for (int r = 0; r < kGramCenterRows; ++r) { cen.x += t[r].x; cen.y += t[r].y; cen.z += t[r].z; cen.w += t[r].w; }
         cen.x *= 0.125f; cen.y *= 0.125f; cen.z *= 0.125f; cen.w *= 0.125f;
       }
-      // Full 16-row groups, branch-free and software-pipelined: the next group's 8 LDS.128 are issued
-      // before this group's 16 STS.64, the 8 independent conversion chains interleave.
-      float4 v[8];
-      if (full_rows > 0) {
-#pragma unroll
-        for (int u = 0; u < 8; ++u) v[u] = lds128(src_lane + static_cast<uint32_t>(2 * u) * 256u);
-      }
-#pragma unroll 1
-      for (int r0 = 0; r0 < full_rows; r0 += 16) {
-        uint32_t h[8][2], l[8][2];
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-          const float x0 = v[u].x - cen.x, x1 = v[u].y - cen.y, x2 = v[u].z - cen.z, x3 = v[u].w - cen.w;
-          h[u][0] = pack_bf16x2_rn(x0, x1);
-          h[u][1] = pack_bf16x2_rn(x2, x3);
-          l[u][0] = pack_bf16x2_rn(x0 - __uint_as_float(h[u][0] << 16), x1 - __uint_as_float(h[u][0] & 0xFFFF0000u));
-          l[u][1] = pack_bf16x2_rn(x2 - __uint_as_float(h[u][1] << 16), x3 - __uint_as_float(h[u][1] & 0xFFFF0000u));
-        }
-        if (r0 + 16 < full_rows) {
-#pragma unroll
-          for (int u = 0; u < 8; ++u) v[u] = lds128(src_lane + static_cast<uint32_t>(r0 + 16 + 2 * u) * 256u);
-        }
-        const uint32_t o0 = static_cast<uint32_t>(r0) * 128u;
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-          const uint32_t off = o0 + static_cast<uint32_t>(u) * 256u + lane_off[u & 3];
-          sts64_u(dst + off, h[u][0], h[u][1]);
-          sts64_u(dst2 + off, l[u][0], l[u][1]);
-        }
-      }
-      if (full_rows < p.n) {                              // ragged tail (n % 16 rows), predicated per row
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-          const int row = full_rows + 2 * u + rsub;
-          if (row < p.n) {
-            float4 t = lds128(src_lane + static_cast<uint32_t>(full_rows + 2 * u) * 256u);
-            t.x -= cen.x; t.y -= cen.y; t.z -= cen.z; t.w -= cen.w;
-            const uint32_t h0 = pack_bf16x2_rn(t.x, t.y), h1 = pack_bf16x2_rn(t.z, t.w);
-            const uint32_t l0 = pack_bf16x2_rn(t.x - __uint_as_float(h0 << 16), t.y - __uint_as_float(h0 & 0xFFFF0000u));
-            const uint32_t l1 = pack_bf16x2_rn(t.z - __uint_as_float(h1 << 16), t.w - __uint_as_float(h1 & 0xFFFF0000u));
-            const uint32_t off = static_cast<uint32_t>(full_rows) * 128u + static_cast<uint32_t>(u) * 256u + lane_off[u & 3];
-            sts64_u(dst + off, h0, h1);
-            sts64_u(dst2 + off, l0, l1);
-          }
-        }
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&raw_empty[w4]);         // done reading this ring slot
+      bf16x2_convert_units(slot, units, src_lane, dst_off, cen);
       fence_proxy_async_smem();
-      named_bar_arrive(1 + w4, 32 + 32);
+      named_bar_arrive(1 + s, 32 + 32);
     }
   } else {
     setmaxnreg_inc<168>();
     // ===================== epilogue: drain TMEM chains into fp32 registers =====================
     const int q = warp & 3;             // TMEM lane quadrant this warp may access
-    const int a = (warp - 8) >> 2;      // 0: b1*b1^T columns, 1: b1*b2^T columns
+    const int a = (warp - 8) >> 2;      // 0: b1*b1^T (8-column groups 2u), 1: b1*b2^T (groups 2u + 1)
+    const uint32_t tmem_base = tmem_base_smem;
     float run[112];
 #pragma unroll
     for (int i = 0; i < 112; ++i) run[i] = 0.f;
@@ -271,15 +189,19 @@ gram_bf16x2_kernel(const __grid_constant__ CUtensorMap tmap, const B16Params p) 
       const int b = g & 1;
       mbar_wait_fast(&acc_full[b], (g >> 1) & 1);
       tc_fence_after();
-      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(b * 256 + a * p.nb);
+      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(b * 256 + a * 8);
 #pragma unroll
-      for (int c = 0; c < 7; ++c) {
-        if (c * 16 < p.nb) {
-          uint32_t v[16];
-          tmem_ld_32x32b_x16(taddr + c * 16, v);
+      for (int u = 0; u < 14; u += 2) {                   // clients 8u .. 8u + 15 (nb is a multiple of 16)
+        if (u * 8 < p.nb) {
+          uint32_t v0[8], v1[8];
+          tmem_ld_32x32b_x8(taddr + u * 16, v0);
+          tmem_ld_32x32b_x8(taddr + u * 16 + 16, v1);
           tmem_ld_wait();
 #pragma unroll
-          for (int i = 0; i < 16; ++i) run[c * 16 + i] += __uint_as_float(v[i]);
+          for (int i = 0; i < 8; ++i) {
+            run[u * 8 + i] += __uint_as_float(v0[i]);
+            run[u * 8 + 8 + i] += __uint_as_float(v1[i]);
+          }
         }
       }
       tc_fence_before();
@@ -297,7 +219,7 @@ gram_bf16x2_kernel(const __grid_constant__ CUtensorMap tmap, const B16Params p) 
   __syncthreads();
   if (warp == 2) {
     tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
+    tmem_dealloc(tmem_base_smem, 512);
   }
 }
 
@@ -336,20 +258,18 @@ int launch_bf16x2(const float* G, int n, int64_t d, int64_t ld, float* parts, in
   p.splits = splits;
   p.parts = parts;
   p.center = center ? 1 : 0;
-  p.cref_rows = n < kGramCenterRows ? n : kGramCenterRows;
-  p.cref = G + static_cast<int64_t>(n - p.cref_rows) * ld;
-  p.cref_ld = ld;
-  p.d = d;
   CUtensorMap tmap;
   const cuuint64_t gdim[2] = {static_cast<cuuint64_t>(d), static_cast<cuuint64_t>(n)};
   const cuuint64_t gstride[1] = {static_cast<cuuint64_t>(ld) * sizeof(float)};
-  const cuuint32_t box[2] = {kB16Cols, static_cast<cuuint32_t>(n)};
+  const cuuint32_t box[2] = {kB16Cols, static_cast<cuuint32_t>(p.nb)};   // rows n..nb-1: zero fill
   const cuuint32_t estride[2] = {1, 1};
   CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(G), gdim, gstride, box, estride,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed: %d", static_cast<int>(r)); return AFL_ERR_CUDA; }
-  const size_t smem = static_cast<size_t>(kRawSlots) * n * 256 + static_cast<size_t>(kBfStages) * p.nb * 256 + 1024;
+  // the last slot's A operand reads kB16ASpan bytes from its base: keep that inside the allocation (+1 KB alignment)
+  const size_t slot_bytes = static_cast<size_t>(p.nb) * 256;
+  const size_t smem = (kB16Slots - 1) * slot_bytes + kB16ASpan + 1024;
   static int smem_attr_done[kMaxDevices] = {0};
   AFL_CUDA(ensure_dyn_smem(gram_bf16x2_kernel, 226 * 1024, smem_attr_done));
   {

@@ -58,37 +58,6 @@ struct PairParams {
                         // no converter pass, no centring), one MMA per 16 columns
 };
 
-__device__ __forceinline__ uint32_t pack_bf16x2_rn_p(float lo, float hi) {
-  uint32_t r;
-  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-  return r;
-}
-__device__ __forceinline__ void sts64_p(uint32_t addr, uint32_t a, uint32_t b) {
-  asm volatile("st.shared.v2.b32 [%0], {%1,%2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
-}
-__device__ __forceinline__ void umma_bf16_p(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// K-major, SWIZZLE_128B, 128-byte rows, 8-row groups `sbo` bytes apart (2048 here: b1 / b2 atoms alternate).
-__device__ __forceinline__ uint64_t umma_desc_sw128_sbo(uint32_t smem_addr, uint32_t sbo) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr & 0x3FFFFu) >> 4);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>(sbo >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(2) << 61;
-  return d;
-}
-__host__ __device__ __forceinline__ uint32_t umma_idesc_bf16_p(uint32_t m, uint32_t n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
-}
-
 __global__ void __launch_bounds__(kPThreads, 1)
 gram_pair_kernel(const __grid_constant__ CUtensorMap tmap, const PairParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -175,7 +144,7 @@ gram_pair_kernel(const __grid_constant__ CUtensorMap tmap, const PairParams p) {
     } else if (warp == 1 || warp == 3) {
       // ===================== MMA issuers (alternating k-blocks) =====================
       const int j = (warp == 3) ? 1 : 0;
-      const uint32_t idesc = umma_idesc_bf16_p(128, 128);
+      const uint32_t idesc = umma_idesc_bf16(128, 128);
       for (int g = 0; g < ngroups; ++g) {
         const int b = g & 1;
         const uint32_t gph = (g >> 1) & 1;
@@ -214,10 +183,10 @@ gram_pair_kernel(const __grid_constant__ CUtensorMap tmap, const PairParams p) {
             for (int ks = 0; ks < 4; ++ks) {             // 4 x K=16 bf16 = 64 columns; +32 bytes per step
               const uint64_t adv = static_cast<uint64_t>(ks * 2);
               const uint32_t acc = (it != it_begin) || (ks != 0);
-              umma_bf16_p(d_hh, d_b1i + adv, d_b1j + adv, idesc, acc);       // hh += b1_I b1_J^T
+              umma_bf16(d_hh, d_b1i + adv, d_b1j + adv, idesc, acc);       // hh += b1_I b1_J^T
               if (!p.in_bf16) {
-                umma_bf16_p(d_x, d_b1i + adv, d_b2j + adv, idesc, acc);      // X  += b1_I b2_J^T
-                umma_bf16_p(d_x, d_b2i + adv, d_b1j + adv, idesc, 1u);       // X  += b2_I b1_J^T
+                umma_bf16(d_x, d_b1i + adv, d_b2j + adv, idesc, acc);      // X  += b1_I b2_J^T
+                umma_bf16(d_x, d_b2i + adv, d_b1j + adv, idesc, 1u);       // X  += b2_I b1_J^T
               }
             }
             umma_commit(&slot_free[s_i]);
@@ -233,19 +202,11 @@ gram_pair_kernel(const __grid_constant__ CUtensorMap tmap, const PairParams p) {
     }
   } else if (wg == 1) {
     setmaxnreg_dec<96>();
-    // ===================== converters: fp32 box -> b1 / b2 atoms, in place =====================
-    // A half warp owns one 256-byte fp32 row (16 lanes x 16 bytes); the warp reads 2 rows per LDS.128 and an
-    // 8-row unit (2 KB) with 4 of them.  The lane with fp32 chunk c16 owns bf16 bytes [8 c16, 8 c16 + 8) of the
-    // 128-byte bf16 row, i.e. half of 16-byte chunk c16/2, which SWIZZLE_128B places at chunk (c16/2)^(row & 7).
+    // ===================== converters: fp32 box -> b1 / b2 atoms, in place (bf16x2_convert_units) =====================
     const int w4 = warp - 4;
-    const int rsub = lane >> 4, c16 = lane & 15;
-    uint32_t dst_off[4];                                  // destination of row 2u + rsub inside the unit
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      const uint32_t row8 = static_cast<uint32_t>(2 * u + rsub);
-      dst_off[u] = row8 * 128u + ((static_cast<uint32_t>(c16 >> 1) ^ row8) << 4) + (static_cast<uint32_t>(c16 & 1) << 3);
-    }
-    const uint32_t src_lane = static_cast<uint32_t>(rsub) * 256u + static_cast<uint32_t>(c16) * 16u;
+    const int c16 = lane & 15;
+    uint32_t src_lane, dst_off[4];
+    bf16x2_lane_offsets(src_lane, dst_off);
     float4 cen = make_float4(0.f, 0.f, 0.f, 0.f);
     auto load_center = [&](int box) -> float4 {
       if (!(p.center && box < nboxes)) return make_float4(0.f, 0.f, 0.f, 0.f);
@@ -257,34 +218,11 @@ gram_pair_kernel(const __grid_constant__ CUtensorMap tmap, const PairParams p) {
       const int s = slot_of(box);
       const uint32_t ph = phase_of(box);
       const float4 cnext = load_center(box + 4);          // in flight while this box is converted
+      // the slot's previous box (another converter's) may still be in flight: wait for its MMA commit first, or the
+      // raw_full wait below could see that box's phase as this one's (see gram_bf16.cu)
+      if (box >= kPSlots) mbar_wait_fast(&slot_free[s], ph ^ 1u);
       mbar_wait_fast(&raw_full[s], ph);
-      const uint32_t base = ring + static_cast<uint32_t>(s) * kPSlotBytes;
-      float4 v[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) v[u] = lds128(base + src_lane + static_cast<uint32_t>(u) * 512u);
-#pragma unroll 1
-      for (int unit = 0; unit < 16; ++unit) {
-        uint32_t h[4][2], l[4][2];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const float x0 = v[u].x - cen.x, x1 = v[u].y - cen.y, x2 = v[u].z - cen.z, x3 = v[u].w - cen.w;
-          h[u][0] = pack_bf16x2_rn_p(x0, x1);
-          h[u][1] = pack_bf16x2_rn_p(x2, x3);
-          l[u][0] = pack_bf16x2_rn_p(x0 - __uint_as_float(h[u][0] << 16), x1 - __uint_as_float(h[u][0] & 0xFFFF0000u));
-          l[u][1] = pack_bf16x2_rn_p(x2 - __uint_as_float(h[u][1] << 16), x3 - __uint_as_float(h[u][1] & 0xFFFF0000u));
-        }
-        const uint32_t ub = base + static_cast<uint32_t>(unit) * 2048u;
-        if (unit + 1 < 16) {                              // next unit's loads before this unit's stores
-#pragma unroll
-          for (int u = 0; u < 4; ++u) v[u] = lds128(ub + 2048u + src_lane + static_cast<uint32_t>(u) * 512u);
-        }
-        __syncwarp();                                     // every lane has read this unit before anyone overwrites it
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          sts64_p(ub + dst_off[u], h[u][0], h[u][1]);
-          sts64_p(ub + 1024u + dst_off[u], l[u][0], l[u][1]);
-        }
-      }
+      bf16x2_convert_units(ring + static_cast<uint32_t>(s) * kPSlotBytes, 16, src_lane, dst_off, cen);
       cen = cnext;
       fence_proxy_async_smem();
       named_bar_arrive(1 + s, 32 + 32);
